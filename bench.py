@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py - packed tokens/s of the TouchNet hot path on B200 (contract: see the task statement / DESIGN.md §6).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
 
 One "step" = one pass of the hot path over one packed synthetic audio+text batch per GPU:
@@ -55,7 +55,12 @@ def parse_args():
                          "kernel writes the bf16 working copies, so this loop has no fp32->bf16 cast kernels")
     ap.add_argument("--no-incumbent", action="store_true",
                     help="skip extras.incumbent (compiled flex_attention / cuBLAS / Liger / HF layer timed next to ours, N=1)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed as DIR/<name>.npy (float32): the loss and a fixed, seeded "
+                         "sample of every parameter gradient, so that two builds can be compared output for output")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     select_workload(args)
     return args
 
@@ -664,6 +669,8 @@ def main():
     tokens_per_step = B * T * dp                     # tp / cp ranks share their rows
     value = dist_util.whole_job_tokens_per_s(B * T, args.steps, dp, ms)
     final_loss = float(loss.item())
+    if args.dump_outputs:                     # before the later arms overwrite the gradients
+        dump_outputs(args.dump_outputs, model, loss, rank)
 
     # ---------------- end-to-end arm: pinned host inputs, H2D inside, loss read back every step ----------------
     e2e = None
@@ -779,6 +786,38 @@ def main():
     print(json.dumps(line), flush=True)
     if dist is not None:
         dist.destroy_process_group()
+
+
+DUMP_SAMPLE = 32768            # gradient elements written per parameter: ~30 MB for the 32-layer workloads
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, model, loss, rank):
+    """What a caller of the timed step receives, as `out_dir/<name>.npy` in float32: `loss` (shape [1]) and
+    `grad.<parameter name>`, the parameter's gradient at DUMP_SAMPLE flat indices drawn with a seed derived from the name
+    (sorted; the whole gradient when it is no larger).  Sharded gradients are gathered first, so every rank calls this;
+    rank 0 writes."""
+    import zlib
+    import numpy as np
+    arrays = {"loss": loss.detach().float().reshape(1).cpu()}
+    for name, p in model.named_parameters():
+        if p.grad is None:
+            continue
+        grad = p.grad.full_tensor() if hasattr(p.grad, "full_tensor") else p.grad
+        flat = grad.detach().reshape(-1)
+        if flat.numel() > DUMP_SAMPLE:
+            g = torch.Generator().manual_seed(zlib.crc32(name.encode()))
+            idx = torch.randint(flat.numel(), (DUMP_SAMPLE,), generator=g).sort().values
+            flat = flat[idx.to(flat.device)]
+        arrays["grad." + name] = flat.float().cpu()
+    if rank != 0:
+        return
+    total = sum(a.numel() * 4 for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit(f"--dump-outputs: {total / 2**20:.1f} MB exceeds {DUMP_LIMIT_BYTES >> 20} MB")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a.numpy())
 
 
 def trace_one_step(step_fn, path, rank, barrier):
